@@ -10,10 +10,14 @@ One "step" = one pass of the hot path over one batch of synthetic input (SURVEY.
 `--impl reference` times the CPU restatement of the reference path (oracle fast path:
   NumPy + SciPy/OpenBLAS, all host threads) on a bounded sample and extrapolates with the
   N^3 / N^2 cost model (the reference is Julia; no julia binary in this image -- DESIGN.md).
+`--dump-outputs DIR` writes what the last timed device step returned (logpdf, posterior mean and
+  variance) as DIR/<name>.npy in float64, so two builds can be compared output for output on the
+  same seeded inputs.
 """
 from __future__ import annotations
 
 import argparse
+import gc
 import json
 import math
 import os
@@ -54,6 +58,26 @@ def make_inputs(n, ns):
     xs = rng.uniform(0, n / 32, ns)
     y = np.sin(x) + 0.3 * rng.standard_normal(n)
     return x, y, xs
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """Write each array as out_dir/<name>.npy (float64).  Outputs larger than DUMP_LIMIT_BYTES in all
+    (only with a large --ns) are replaced by the same fixed, seeded sample of entries, whose indices
+    are written too as sample_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        size = max(a.size for a in arrays.values())
+        keep = size * DUMP_LIMIT_BYTES // (2 * total)  # half the budget: leaves room for the index
+        idx = np.sort(np.random.default_rng(0).choice(size, keep, replace=False))
+        arrays = {k: a[idx] if a.size == size else a for k, a in arrays.items()}
+        arrays["sample_index"] = idx.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -316,14 +340,18 @@ def gpu_main(args):
         m, v = sb.mean_and_var(post, sb.GPPPInput("f", xs))
         return lp, m, v
 
-    e2e_steps = max(1, min(args.steps, 2))
     e2e_step()
-    barrier()
-    t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    e2e_s = 0.0
+    for _ in range(args.steps):
+        # A posterior and its factor refer to each other, so the previous step's device factor
+        # (17 GB at N = 65536) is freed only by the cycle collector: free it before the next step.
+        gc.collect()
+        barrier()
+        t0 = time.perf_counter()
         lp_e, m_e, v_e = e2e_step()
-    torch.cuda.synchronize()
-    e2e_s = (time.perf_counter() - t0) / e2e_steps
+        torch.cuda.synchronize()
+        e2e_s += time.perf_counter() - t0
+    e2e_s /= args.steps
     if dist is not None:
         tt = torch.tensor([e2e_s], dtype=torch.float64)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -344,6 +372,8 @@ def gpu_main(args):
         shutdown()
         return
     mean_h, var_h = mean_d.cpu().numpy(), var_d.cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, logpdf=np.float64(lp), mean=mean_h, var=var_h)
     np.testing.assert_allclose(mean_h, m_e, rtol=1e-9, atol=1e-10)
     # ---- parity against the committed single-GPU result of the same seeded inputs -----------------
     # (tests/golden/config2_n1.json: written by a 1-GPU DMMA run, itself oracle-checked at N <= 32768
@@ -485,7 +515,13 @@ def main():
     ap.add_argument("--write-golden", action="store_true", help="(1 GPU) rewrite tests/golden/config2_n1.json")
     ap.add_argument("--trailing", default=os.environ.get("SB_BENCH_TRAILING", DEFAULT_TRAILING), choices=["dmma", "ozaki"],
                     help="Cholesky trailing update: fp64 DMMA (mma.sync) or tcgen05 int8 Ozaki slices")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="(b200) write the last timed step's logpdf, posterior mean and variance as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the device path: use it with --impl b200")
     global _OUT_FD
     sys.stdout.flush()
     _OUT_FD = os.dup(1)

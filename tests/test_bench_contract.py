@@ -43,6 +43,31 @@ def test_extrapolation_model():
     assert np.isclose(bench.cpu_extrapolate(t, 100, 10, 100, 20), 1 + 2 + 0.5 + 6)
 
 
+def test_dump_outputs_float64_and_bounded_sample(tmp_path, monkeypatch):
+    import bench
+    mean, var = np.arange(1000, dtype=np.float64), np.arange(1000, dtype=np.float32) * 0.5
+    bench.dump_outputs(str(tmp_path / "full"), logpdf=np.float64(-3.5), mean=mean, var=var)
+    got = {p.stem: np.load(p) for p in (tmp_path / "full").iterdir()}
+    assert sorted(got) == ["logpdf", "mean", "var"] and all(a.dtype == np.float64 for a in got.values())
+    assert got["logpdf"] == -3.5 and np.array_equal(got["mean"], mean) and np.array_equal(got["var"], var)
+    # above the limit: the same seeded sample of entries every time, within the limit, indices included
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), logpdf=np.float64(-3.5), mean=mean, var=var)
+    a, b = ({p.stem: np.load(p) for p in (tmp_path / d).iterdir()} for d in ("a", "b"))
+    assert sorted(a) == ["logpdf", "mean", "sample_index", "var"]
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert sum(v.nbytes for v in a.values()) <= 4000
+    idx = a["sample_index"].astype(np.int64)
+    assert np.array_equal(a["mean"], mean[idx]) and np.array_equal(a["var"], var[idx])
+
+
+def test_bench_rejects_zero_steps():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_committed_gpu_bench_line_has_contract_keys():
     d = json.loads(open(os.path.join(ROOT, "profiles", "bench_r1_1gpu.json")).read().strip().splitlines()[-1])
     for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
