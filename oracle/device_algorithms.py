@@ -7,6 +7,10 @@ LAPACK / exact arithmetic and the CUDA sources can cite a runnable specification
 
   * `oz_slice`, `oz_product`      -- the int8 digit-plane ("Ozaki") product of stheno.jl_b200/csrc/ozaki.cu
                                      (oz_rowscale_kernel, oz_slice_kernel, the 7 grouped int32 accumulators);
+  * `oz_groups`, `oz_epilogue_acc`, `oz_update`, `oz_store`, `oz_syrk_tiles`, the packed-layout helpers
+                                  -- the same product restated bit for bit as the tcgen05 kernel computes it
+                                     (accumulators, epilogue rounding order, the tiles a launch covers), so that
+                                     tests/test_gpu_ozaki_exact.py can demand equality of every output bit;
   * `wide_panel_factor`           -- the wide panel phase of api.cu (wide_diag_phase + launch_panel_solve_ozaki):
                                      512 x 512 diagonal block stacked over an identity, right-looking 128-block
                                      elimination, X = A inv(L_512)^T for the rows below;
@@ -29,6 +33,17 @@ NB = 128
 # ---------------------------------------------------------------------------------------------------------
 # int8 digit planes
 # ---------------------------------------------------------------------------------------------------------
+OZ_NO_EXPO = 0x7fffffff   # exponent the slicer stores for a row it maps to zero digits
+
+
+def oz_row_exponents(P: np.ndarray) -> np.ndarray:
+    """Row exponents e_i = ilogb(max|P[i, :]|) + 2 as oz_rowscale_kernel stores them: OZ_NO_EXPO for a row whose
+    max is not inside (1e-280, 1e280) (all zero, tiny or huge rows get zero digits and scale 0)."""
+    mx = np.max(np.abs(np.asarray(P, dtype=np.float64)), axis=1)
+    ok = (mx > 1e-280) & (mx < 1e280)
+    return np.where(ok, np.frexp(np.where(ok, mx, 1.0))[1] - 1 + 2, OZ_NO_EXPO).astype(np.int32)
+
+
 def oz_slice(P: np.ndarray):
     """Digit planes of the rows of P (m x K).  Returns (digits[7, m, K] int8, scale[m] float64).
 
@@ -40,9 +55,9 @@ def oz_slice(P: np.ndarray):
     """
     P = np.asarray(P, dtype=np.float64)
     m, K = P.shape
-    mx = np.max(np.abs(P), axis=1)
-    ok = (mx > 1e-280) & (mx < 1e280)
-    e = np.where(ok, np.frexp(np.where(ok, mx, 1.0))[1] - 1 + 2, 0)      # ilogb(m) + 2
+    expo = oz_row_exponents(P)
+    ok = expo != OZ_NO_EXPO
+    e = np.where(ok, expo, 0)
     scale = np.where(ok, np.ldexp(1.0, e - 31), 0.0)
     Z = np.zeros((m, K), dtype=np.int64)
     Z[ok] = np.rint(np.ldexp(P[ok], (55 - e[ok])[:, None])).astype(np.int64)
@@ -81,6 +96,100 @@ def oz_product(dA, sA, dB, sB, max_group: int = OZ_S - 1):
     # x = s 2^-24 sum d_p 256^(6-p)  ->  x_i x_j = s_i s_j 2^-48 sum_g 256^(12-g) G_g; the kernel's s already
     # absorbs 2^-24 * 256^3 per operand (s = 2^(e-31) = 2^(e-55) 256^3), leaving 256^(6-g)
     return acc * sA[:, None] * sB[None, :], gmax
+
+
+# ---------------------------------------------------------------------------------------------------------
+# the tcgen05 kernel, bit for bit
+# ---------------------------------------------------------------------------------------------------------
+def oz_groups(dA: np.ndarray, dB: np.ndarray) -> list:
+    """The seven int32 accumulators G_g = sum_{p+q=g} d_p(A) d_q(B)^T, g = 0..6, as float64 arrays of exact
+    integers.  One float64 BLAS product per group on the int8-valued digits (the pairs of a group are concatenated
+    along K): every partial sum is an integer of magnitude below 7 * 512 * 2^14 < 2^53, so the result is exact
+    whatever order the BLAS sums in."""
+    A = dA.astype(np.float64)
+    B = dB.astype(np.float64)
+    return [np.concatenate([A[p] for p in range(g + 1)], axis=1) @
+            np.concatenate([B[g - p] for p in range(g + 1)], axis=1).T for g in range(OZ_S)]
+
+
+def oz_epilogue_acc(G: list) -> np.ndarray:
+    """The epilogue's fp64 sum: acc = fma((double)G_g, 2^(8(6 - g)), acc) for g = 0..6 in this order.  The product
+    is exact, so each step is one rounding of acc + G_g 2^(8(6 - g)), which is what NumPy's addition does."""
+    acc = np.zeros_like(G[0])
+    for g in range(OZ_S):
+        acc = acc + G[g] * math.ldexp(1.0, 8 * (OZ_S - 1 - g))
+    return acc
+
+
+def oz_update(old: np.ndarray, sA: np.ndarray, sB: np.ndarray, acc: np.ndarray) -> np.ndarray:
+    """SYRK / plain mode: C = fma(-(s_i s_j), acc, C), with s_i s_j formed first.  s_i s_j is a power of two (or 0),
+    so the product with acc is exact and old - s_i s_j acc rounds once like the fma, as long as the product stays
+    in the normal range (asserted: below it the fma's single rounding is not what NumPy computes)."""
+    s = sA[:, None] * sB[None, :]
+    p = s * acc
+    assert not np.any((np.abs(p) < np.finfo(np.float64).tiny) & (s != 0) & (acc != 0)), "product below the normal range"
+    return old - p
+
+
+def oz_store(sA: np.ndarray, sB: np.ndarray, acc: np.ndarray) -> np.ndarray:
+    """STORE mode (panel solve): X = (s_i s_j) acc."""
+    return (sA[:, None] * sB[None, :]) * acc
+
+
+def packed_offset(Np: int, J: int) -> int:
+    """Element offset of block column J in the packed lower layout (sb_common.cuh `Packed`)."""
+    return NB * (J * Np - NB * (J * (J - 1) // 2))
+
+
+def packed_size(Np: int) -> int:
+    return packed_offset(Np, Np // NB)
+
+
+def packed_column(buf: np.ndarray, Np: int, J: int) -> np.ndarray:
+    """Writable (Np - J NB) x NB view of block column J (rows J NB .. Np - 1) of a packed buffer."""
+    ld = Np - J * NB
+    o = packed_offset(Np, J)
+    return buf[o:o + NB * ld].reshape(NB, ld).T
+
+
+def tiled_offset(rb: int, k: int, r: int) -> int:
+    """Element (row block rb, column k, row r) of a TILED panel buffer: [row block][128 columns][132 padded rows]."""
+    return (rb * NB + k) * (NB + 4) + r
+
+
+def oz_syrk_tiles(nblk: int, k: int, jlo: int, jhi: int, rank: int = 0, world: int = 1,
+                  tile_lo: int = 0, tile_hi: int = 0) -> list:
+    """(I, J, h) of the 128 x 64 tiles launch_syrk_ozaki updates, in the kernel's tile order (OzCursor): owned block
+    columns J = J0, J0 + world, ... in [max(jlo, k + 1), jhi) with J % world == rank, in each the row blocks I >= J,
+    in each both 64-column halves h.  tile_lo / tile_hi select a sub-range of the list; tile_hi <= 0 means its end."""
+    jlo, jhi = max(jlo, k + 1), min(jhi, nblk)
+    J0 = jlo + (rank - jlo) % world
+    tiles = [(I, J, h) for J in range(J0, jhi, world) for I in range(J, nblk) for h in (0, 1)]
+    if tile_hi <= 0 or tile_hi > len(tiles):
+        tile_hi = len(tiles)
+    return tiles[max(tile_lo, 0):tile_hi]
+
+
+def oz_syrk_update(packed: np.ndarray, Np: int, digits: np.ndarray, scale: np.ndarray) -> np.ndarray:
+    """The packed matrix with EVERY block (I >= J) updated as the SYRK instance updates a tile of it:
+    C -= P P^T from the digit planes digits[7][Np][K] and scales[Np] of the rows (plane row == matrix row), the
+    strictly upper part of the diagonal blocks included.  Combine with oz_apply_tiles for what one launch writes."""
+    out = packed.copy()
+    for J in range(Np // NB):
+        r0 = J * NB
+        acc = oz_epilogue_acc(oz_groups(digits[:, r0:], digits[:, r0:r0 + NB]))
+        V = packed_column(out, Np, J)
+        V[...] = oz_update(V, scale[r0:], scale[r0:r0 + NB], acc)
+    return out
+
+
+def oz_apply_tiles(old: np.ndarray, new: np.ndarray, Np: int, tiles) -> np.ndarray:
+    """`old` with the tiles (I, J, h) taken from `new`."""
+    out = old.copy()
+    for I, J, h in tiles:
+        rows, cols = slice((I - J) * NB, (I - J + 1) * NB), slice(h * 64, h * 64 + 64)
+        packed_column(out, Np, J)[rows, cols] = packed_column(new, Np, J)[rows, cols]
+    return out
 
 
 # ---------------------------------------------------------------------------------------------------------

@@ -2,7 +2,9 @@
 `cholesky(Symmetric(cov(fx)))`, SURVEY.md App. A): the int8 digit-plane product, the wide panel phase and the
 peer-to-peer exchange protocol -- restated in NumPy in oracle/device_algorithms.py and checked here against
 exact integer arithmetic, LAPACK and randomised interleavings.  The device kernels are compared with the same
-quantities on the GPU (tools/oz_test.cu: exact digit products; tests/test_gpu_parity.py: the oracle)."""
+quantities on the GPU: tests/test_gpu_ozaki_exact.py demands bit-for-bit equality of every tcgen05 kernel instance
+with the exact model pinned here; tests/test_gpu_parity.py compares the whole pipeline with the oracle."""
+import math
 from fractions import Fraction
 
 import numpy as np
@@ -137,3 +139,101 @@ def test_p2p_exchange_without_the_slot_guard_is_caught():
             assert "overwrites slot" in str(e) or "expected column" in str(e)
             hit += 1
     assert hit > 0
+
+
+def test_blas_groups_equal_the_int64_accumulators():
+    """oz_groups (float64 BLAS on the int8 digits) is exact: it equals the int64 sums of oz_product's loop."""
+    rng = np.random.default_rng(8)
+    dA, _ = da.oz_slice(_rows(rng, 40, 512, 10.0))
+    dB, _ = da.oz_slice(_rows(rng, 24, 512, 10.0))
+    dA[1:, :3] = -128                               # extreme digits in a few columns
+    dB[1:, :3] = -128
+    G = da.oz_groups(dA, dB)
+    for g in range(7):
+        ref = sum(dA[p].astype(np.int64) @ dB[g - p].astype(np.int64).T for p in range(g + 1))
+        assert np.array_equal(G[g].astype(np.int64), ref) and np.array_equal(G[g], ref.astype(np.float64))
+
+
+def test_epilogue_model_agrees_with_the_digit_plane_product():
+    """The epilogue-ordered model (groups -> weighted fp64 sum -> (s_i s_j) acc) is oz_product bit for bit on rows
+    of normal magnitude, and the SYRK update is C - that product rounded once."""
+    rng = np.random.default_rng(9)
+    A, B = _rows(rng, 32, 384, 6.0), _rows(rng, 20, 384, 6.0)
+    A[3] = 0.0
+    dA, sA = da.oz_slice(A)
+    dB, sB = da.oz_slice(B)
+    acc = da.oz_epilogue_acc(da.oz_groups(dA, dB))
+    X = da.oz_store(sA, sB, acc)
+    assert np.array_equal(X.view(np.int64), da.oz_product(dA, sA, dB, sB)[0].view(np.int64))
+    C = rng.standard_normal((32, 20))
+    assert np.array_equal(da.oz_update(C, sA, sB, acc), C - X)
+
+
+def test_slicer_exponents_at_the_ilogb_and_range_boundaries():
+    P = np.zeros((6, 4))
+    P[0, 1] = 8.0                                   # max exactly 2^3: e = 3 + 2
+    P[1, 2] = np.nextafter(8.0, 0.0)                # 2^3 - ulp: e = 2 + 2
+    P[2, 0] = -8.0                                  # negative maximum
+    P[3, 3] = 1e-280                                # not above 1e-280: zero row
+    P[4, 3] = np.nextafter(1e-280, 1.0)
+    P[5, 0] = np.nextafter(1e280, 0.0)
+    e = da.oz_row_exponents(P)
+    assert list(e[:3]) == [5, 4, 5] and e[3] == da.OZ_NO_EXPO
+    assert e[4] == int(np.frexp(1e-280)[1]) + 1 and e[5] == int(np.frexp(1e280)[1]) + 1
+
+
+def test_headroom_rows_give_extreme_digits():
+    """Z = 64 2^48 - 0x808080808080 slices to d_0 = 64 and six digits -128 (the largest digits a row can have);
+    Z = -63 2^48 - 0x808080808080 to d_0 = -63 and six digits -128."""
+    bias = 0x808080808080
+    for d0 in (64, -63):
+        Z = d0 * 2 ** 48 - bias
+        x = np.full((1, 8), math.ldexp(float(Z), 1 - 55))          # e = 1
+        d, s = da.oz_slice(x)
+        assert s[0] == 2.0 ** -30 and np.all(d[0] == d0) and np.all(d[1:] == -128)
+
+
+def test_syrk_tile_set_follows_the_launcher():
+    nblk = 12
+    for k, jlo, jhi in [(0, 0, nblk), (2, 0, 7), (0, 5, 6), (3, 9, 30)]:
+        full = da.oz_syrk_tiles(nblk, k, jlo, jhi)
+        lo, hi = max(jlo, k + 1), min(jhi, nblk)
+        assert len(full) == 2 * sum(nblk - J for J in range(lo, hi))
+        assert full == sorted(full, key=lambda t: (t[1], t[0], t[2]))
+        for world in (2, 3):
+            parts = [da.oz_syrk_tiles(nblk, k, jlo, jhi, r, world) for r in range(world)]
+            assert sorted(sum(parts, [])) == sorted(full)
+            assert all(J % world == r for r, part in enumerate(parts) for _, J, _ in part)
+        n1 = len(full) // 3
+        assert da.oz_syrk_tiles(nblk, k, jlo, jhi, tile_hi=n1) + da.oz_syrk_tiles(nblk, k, jlo, jhi, tile_lo=n1) == full
+
+
+def test_packed_layout_helpers():
+    Np = 512
+    buf = np.arange(da.packed_size(Np), dtype=np.float64)
+    assert da.packed_size(Np) == Np * (Np + 128) // 2
+    for J in range(Np // 128):
+        V = da.packed_column(buf, Np, J)
+        ld = Np - 128 * J
+        assert V.shape == (ld, 128)
+        assert V[5, 7] == da.packed_offset(Np, J) + 7 * ld + 5
+
+
+def test_syrk_model_is_the_lower_triangle_of_the_dense_update():
+    rng = np.random.default_rng(10)
+    Np, K = 384, 256
+    P = _rows(rng, Np, K, 4.0)
+    d, s = da.oz_slice(P)
+    C = rng.standard_normal(da.packed_size(Np))
+    new = da.oz_syrk_update(C, Np, d, s)
+    dense = da.oz_store(s, s, da.oz_epilogue_acc(da.oz_groups(d, d)))
+    for J in range(3):
+        r0 = 128 * J
+        want = da.packed_column(C, Np, J) - dense[r0:, r0:r0 + 128]
+        assert np.array_equal(da.packed_column(new, Np, J), want)
+    half = da.oz_syrk_tiles(3, 0, 0, 3, tile_hi=3)            # (1, 1, 0), (1, 1, 1), (2, 1, 0)
+    part = da.oz_apply_tiles(C, new, Np, half)
+    V, Vn = da.packed_column(part, Np, 1), da.packed_column(new, Np, 1)
+    assert np.array_equal(V[:, :64], Vn[:, :64]) and np.array_equal(V[:128, 64:], Vn[:128, 64:])
+    assert np.array_equal(V[128:, 64:], da.packed_column(C, Np, 1)[128:, 64:])
+    assert np.array_equal(da.packed_column(part, Np, 0), da.packed_column(C, Np, 0))

@@ -527,13 +527,21 @@ def ozaki_ctx(sb):
         ctx.set_option("trailing", DEFAULT_TRAILING)
 
 
-@pytest.mark.parametrize("n", [2500, 4096])
+# Test points per size; the sizes below 2500 end the factorisation with a short outer step:
+# nblk = ceil(N / 128) = 9, 10, 11, 13 leaves nq = 1, 2, 3, 1 block columns (1663: N % 128 = 127).
+OZ_TEST_POINTS = {1025: 1, 1153: 127, 1281: 129}
+OZ_MODES = [0, 2, 4, 6, 8, 10, 16]   # the tcgen05 variants SB_OZ_MODE accepts; 2, 6, 10 factor by look-ahead
+OZ_DEFAULT_MODE = 8
+
+
+@pytest.mark.parametrize("n", [2500, 4096, 1025, 1153, 1281, 1663])
 def test_tcgen05_ozaki_trailing_update_parity(sb, orc, ozaki_ctx, n):
     """fp64 Cholesky whose trailing SYRK runs as 28 int8 tcgen05 MMAs per fp64 MMA (ozaki.cu):
-    the factor must agree with LAPACK to 1e-12 and logpdf / posterior with the oracle to 1e-10."""
+    the factor must agree with LAPACK to 1e-12 and logpdf / posterior with the oracle to 1e-10.
+    At N = 1153 logpdf and posterior are also checked under every kernel variant (oz_mode)."""
     import scipy.linalg as sla
     rng = np.random.default_rng(41)
-    x, xs = rng.uniform(0, n / 32, n), rng.uniform(0, n / 32, 300)
+    x, xs = rng.uniform(0, n / 32, n), rng.uniform(0, n / 32, OZ_TEST_POINTS.get(n, 300))
     y = np.sin(x) + 0.3 * rng.standard_normal(n)
     fs, fo = sb.gppp(lambda GP: dict(f=GP(sb.SEKernel()))), orc.gppp(lambda GP: dict(f=GP(orc.SEKernel())))
     fxs, fxo = fs(sb.GPPPInput("f", x), 0.1), fo(orc.GPPPInput("f", x), 0.1)
@@ -549,6 +557,21 @@ def test_tcgen05_ozaki_trailing_update_parity(sb, orc, ozaki_ctx, n):
     mo, vo = orc.mean_and_var(orc.posterior(fxo, y), orc.GPPPInput("f", xs))
     np.testing.assert_allclose(m, mo, rtol=RTOL, atol=1e-11)
     np.testing.assert_allclose(v, vo, rtol=RTOL, atol=1e-11)
+    if n != 1153:
+        return
+    try:
+        for mode in OZ_MODES:
+            ozaki_ctx.set_option("oz_mode", mode)
+            ozaki_ctx.timings(reset=True)
+            fxm = fs(sb.GPPPInput("f", x), 0.1)
+            lp = sb.logpdf(fxm, y)
+            assert ozaki_ctx.timings()["trailing_int8_ops"] > 0, f"oz_mode {mode}: the tcgen05 path did not run"
+            assert abs(lp - lpo) <= RTOL * abs(lpo), (mode, lp, lpo)
+            m, v = sb.mean_and_var(sb.posterior(fxm, y), sb.GPPPInput("f", xs))
+            np.testing.assert_allclose(m, mo, rtol=RTOL, atol=1e-11, err_msg=f"oz_mode {mode}")
+            np.testing.assert_allclose(v, vo, rtol=RTOL, atol=1e-11, err_msg=f"oz_mode {mode}")
+    finally:
+        ozaki_ctx.set_option("oz_mode", OZ_DEFAULT_MODE)
 
 
 def test_dmma_trailing_update_parity(sb, orc):

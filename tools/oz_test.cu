@@ -1,7 +1,8 @@
-// Standalone check + timing of the tcgen05 int8-Ozaki trailing update (stheno.jl_b200/csrc/ozaki.cu)
-// against (a) exact integer digit products computed on the CPU for one tile and (b) the fp64 DMMA
-// trailing kernel (gemm_nt.cu) on the whole trailing matrix.  Build: tools/Makefile (links build/*.o).
-//   oz_test [Np=4096] [timing_Np=0] [nseg=4]
+// Standalone timing of the tcgen05 int8-Ozaki trailing update (stheno.jl_b200/csrc/ozaki.cu) next to the
+// fp64 DMMA trailing kernel (gemm_nt.cu) on the same panels.  Correctness of every kernel instance is
+// tests/test_gpu_ozaki_exact.py (bit-for-bit against the exact model).  Build: tools/Makefile (links build/*.o).
+//   oz_test [Np=16384] [nseg=4]     (OZ_TEST_RESERVE: see below)
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -22,7 +23,6 @@ static double urand(uint64_t& s) {
 struct Problem {
     int64_t Np, nblk, k0;
     int nseg;
-    std::vector<double> hP[4];
     double* dP[4] = {nullptr, nullptr, nullptr, nullptr};
     const double** dPt = nullptr;  // device array of panel pointers
     double *A1 = nullptr, *A2 = nullptr;
@@ -32,12 +32,13 @@ struct Problem {
     Packed P1, P2;
 };
 
-static int setup(Problem& pr, int64_t Np, int nseg, bool host_copy) {
+static int setup(Problem& pr, int64_t Np, int nseg) {
     pr.Np = Np; pr.nblk = Np / NB; pr.k0 = 0; pr.nseg = nseg;
     const int64_t pe = tiled_panel_elems(Np);
     uint64_t seed = 12345;
+    std::vector<double> hP(pe);
     for (int q = 0; q < nseg; q++) {
-        pr.hP[q].assign(pe, 0.0);
+        std::fill(hP.begin(), hP.end(), 0.0);
         for (int64_t rb = 0; rb < pr.nblk; rb++)
             for (int k = 0; k < NB; k++)
                 for (int r = 0; r < NB; r++) {
@@ -45,11 +46,10 @@ static int setup(Problem& pr, int64_t Np, int nseg, bool host_copy) {
                     double mag = std::pow(10.0, -3.0 * ((rb * NB + r) % 7) / 7.0) * ((r % 13 == 5) ? 1e-6 : 1.0);
                     double v = (urand(seed) * 2 - 1) * mag;
                     if ((r + k) % 97 == 0) v = 0.0;
-                    pr.hP[q][((rb * NB + k) * (int64_t)(NB + 4)) + r] = v;
+                    hP[((rb * NB + k) * (int64_t)(NB + 4)) + r] = v;
                 }
         CK(cudaMalloc(&pr.dP[q], pe * 8));
-        CK(cudaMemcpy(pr.dP[q], pr.hP[q].data(), pe * 8, cudaMemcpyHostToDevice));
-        if (!host_copy) { pr.hP[q].clear(); pr.hP[q].shrink_to_fit(); }
+        CK(cudaMemcpy(pr.dP[q], hP.data(), pe * 8, cudaMemcpyHostToDevice));
     }
     CK(cudaMalloc(&pr.dPt, 4 * sizeof(double*)));
     CK(cudaMemcpy(pr.dPt, pr.dP, 4 * sizeof(double*), cudaMemcpyHostToDevice));
@@ -77,137 +77,18 @@ static void teardown(Problem& pr) {
     cudaFree(pr.dPt); cudaFree(pr.A1); cudaFree(pr.A2); cudaFree(pr.scale); cudaFree(pr.expo); cudaFree(pr.planes);
 }
 
-// CPU digits of row (global row i) for the K = 128*nseg columns
-static void cpu_digits(const Problem& pr, int64_t i, std::vector<int>& d /*[7][K]*/, double& scale) {
-    const int K = 128 * pr.nseg;
-    d.assign(7 * K, 0);
-    const int64_t rb = i / NB - pr.k0 - 1;
-    const int r = (int)(i % NB);
-    double m = 0;
-    for (int q = 0; q < pr.nseg; q++)
-        for (int k = 0; k < NB; k++) m = std::fmax(m, std::fabs(pr.hP[q][((rb * NB + k) * (int64_t)(NB + 4)) + r]));
-    if (!(m > 1e-280)) { scale = 0; return; }
-    const int e = std::ilogb(m) + 2;
-    scale = std::scalbn(1.0, e - 31);
-    for (int q = 0; q < pr.nseg; q++)
-        for (int k = 0; k < NB; k++) {
-            double x = pr.hP[q][((rb * NB + k) * (int64_t)(NB + 4)) + r];
-            long long Z = 0x0000808080808080LL + std::llrint(std::scalbn(x, 55 - e));
-            d[0 * K + q * NB + k] = (int)(signed char)(Z >> 48);
-            for (int p = 1; p < 7; p++) d[p * K + q * NB + k] = (int)(signed char)(((Z >> (8 * (6 - p))) & 0xff) ^ 0x80);
-        }
-}
-
 // OZ_TEST_RESERVE: > 0 leaves that many SMs free (persistent grid), < 0 launches chunked CTAs of -value tiles
 static int g_reserve = 0;
 
 int main(int argc, char** argv) {
     if (getenv("OZ_TEST_RESERVE")) g_reserve = atoi(getenv("OZ_TEST_RESERVE"));
-    const int64_t Np = argc > 1 ? atoll(argv[1]) : 4096;
-    const int64_t NpT = argc > 2 ? atoll(argv[2]) : 0;
-    const int nseg = argc > 3 ? atoi(argv[3]) : 4;
+    const int64_t NpT = argc > 1 ? atoll(argv[1]) : 16384;
+    const int nseg = argc > 2 ? atoi(argv[2]) : 4;
     cudaStream_t st;
     CK(cudaStreamCreate(&st));
     {
         Problem pr;
-        if (setup(pr, Np, nseg, true)) return 1;
-        const int64_t jt = nseg;
-        // reference: DMMA kernel
-        const double* Pt[4] = {pr.dP[0], pr.dP[1], pr.dP[2], pr.dP[3]};
-        launch_syrk_packed(pr.P1, 0, Pt, nseg, jt, pr.nblk, 0, 1, st);
-        CK(cudaStreamSynchronize(st));
-        const int64_t tot = pr.P1.total();
-        std::vector<double> h0(tot), h1(tot), h2(tot);
-        CK(cudaMemcpy(h1.data(), pr.A1, tot * 8, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(h0.data(), pr.A2, tot * 8, cudaMemcpyDeviceToHost));  // original C
-
-        launch_oz_slice(oz_src_tiled(Pt, nseg), nseg - 1, pr.nblk - nseg, (int64_t)NB, Np, pr.scale, pr.expo, pr.planes, st);
-        CK(cudaStreamSynchronize(st));
-        CK(cudaGetLastError());
-        // check the digit planes of one row against the CPU
-        {
-            const int64_t i = jt * NB + 37;
-            std::vector<int> d; double sc;
-            cpu_digits(pr, i, d, sc);
-            std::vector<signed char> hp(7 * 512);
-            for (int p = 0; p < 7; p++)
-                CK(cudaMemcpy(hp.data() + p * 512, pr.planes + ((int64_t)p * Np + i) * 512, 512, cudaMemcpyDeviceToHost));
-            double hs;
-            CK(cudaMemcpy(&hs, pr.scale + i, 8, cudaMemcpyDeviceToHost));
-            int bad = 0;
-            for (int p = 0; p < 7; p++) for (int k = 0; k < 128 * nseg; k++) bad += (hp[p * 512 + k] != d[p * 128 * nseg + k]);
-            printf("[slice] row %lld: digit mismatches %d, scale dev %.6e cpu %.6e\n", (long long)i, bad, hs, sc);
-        }
-        int* dbg = nullptr;
-        CK(cudaMalloc(&dbg, 7 * 128 * 64 * 4));
-
-        struct Variant { const char* name; int tma_mode; int lbo_override; int sbo_override; };
-        // (round 2: all three encodings below reproduce the CPU digit products exactly on B200; the
-        //  LBO field is indeed ignored for swizzled K-major operands)
-        Variant vars[] = {{"sw64 x2 stages", 0, -1, -1}, {"sw32 x5 stages", 2, -1, -1}, {"interleave default", 1, -1, -1},
-                          {"sw64 x2, A via TMEM", 4, -1, -1}, {"sw32 x5, A via TMEM", 6, -1, -1},
-                          {"sw64 x2, paired N=128", 8, -1, -1}, {"sw32 x5, paired N=128", 10, -1, -1},
-                          {"ring: 18 A-plane slots, paired N", 16, -1, -1}, {"sw64 x2, A via TMEM + paired N", 12, -1, -1}};
-        for (auto& v : vars) {
-            CK(cudaMemcpy(pr.A2, h0.data(), tot * 8, cudaMemcpyHostToDevice));
-            CK(cudaMemset(dbg, 0xff, 7 * 128 * 64 * 4));
-            OzMaps maps;
-            if (oz_make_maps(pr.planes, Np, v.tma_mode, &maps)) { printf("[%s] tensor map creation failed\n", v.name); continue; }
-            OzDesc d;
-            oz_default_desc(&d, v.tma_mode);
-            if (v.lbo_override >= 0) d.a_lbo = d.b_lbo = v.lbo_override;
-            if (v.lbo_override == -2) { uint32_t a = d.a_lbo, b = d.b_lbo; d.a_lbo = d.b_lbo = d.sbo; d.sbo = a; (void)b; }
-            int rc = launch_syrk_ozaki(pr.P2, 0, nseg, jt, pr.nblk, 0, 1, &maps, pr.scale, &d, v.tma_mode, st, g_reserve, dbg);
-            cudaError_t e = cudaStreamSynchronize(st);
-            if (rc || e != cudaSuccess) {
-                printf("[%s] launch rc=%d, cuda: %s\n", v.name, rc, cudaGetErrorString(e));
-                return 2;  // context is dead after a trap
-            }
-            // (a) exact integer check of tile 0: I = J = jt, h = 0
-            std::vector<int> hd(7 * 128 * 64);
-            CK(cudaMemcpy(hd.data(), dbg, hd.size() * 4, cudaMemcpyDeviceToHost));
-            const int K = 128 * nseg;
-            std::vector<std::vector<int>> dig(128);
-            std::vector<double> sc(128);
-            for (int r = 0; r < 128; r++) cpu_digits(pr, jt * NB + r, dig[r], sc[r]);
-            long long nbad = 0; int shown = 0;
-            for (int grp = 0; grp < 7; grp++)
-                for (int r = 0; r < 128; r++)
-                    for (int c = 0; c < 64; c++) {
-                        long long G = 0;
-                        for (int p = 0; p <= grp; p++) {
-                            const int q = grp - p;
-                            const int* a = &dig[r][p * K];
-                            const int* b = &dig[c][q * K];
-                            for (int k = 0; k < K; k++) G += (long long)a[k] * b[k];
-                        }
-                        int got = hd[(grp * 128 + r) * 64 + c];
-                        if ((long long)got != G) {
-                            nbad++;
-                            if (shown < 6) { printf("   grp %d r %d c %d: got %d want %lld\n", grp, r, c, got, G); shown++; }
-                        }
-                    }
-            // (b) whole trailing matrix vs DMMA
-            CK(cudaMemcpy(h2.data(), pr.A2, tot * 8, cudaMemcpyDeviceToHost));
-            double maxd = 0, maxref = 0;
-            for (int64_t J = jt; J < pr.nblk; J++)
-                for (int64_t I = J; I < pr.nblk; I++)
-                    for (int c = 0; c < NB; c++)
-                        for (int r = 0; r < NB; r++) {
-                            if (I == J && r < c) continue;
-                            int64_t off = (pr.P1.blk(I, J) - pr.P1.base) + (int64_t)c * pr.P1.ld(J) + r;
-                            maxd = std::fmax(maxd, std::fabs(h1[off] - h2[off]));
-                            maxref = std::fmax(maxref, std::fabs(h1[off] - h0[off]));
-                        }
-            printf("[%s] tile-0 integer mismatches: %lld / %d ; trailing max|ozaki - dmma| = %.3e (update magnitude %.3e)\n",
-                   v.name, nbad, 7 * 128 * 64, maxd, maxref);
-        }
-        cudaFree(dbg);
-        teardown(pr);
-    }
-    if (NpT > 0) {
-        Problem pr;
-        if (setup(pr, NpT, nseg, false)) return 1;
+        if (setup(pr, NpT, nseg)) return 1;
         const int64_t jt = nseg;
         const double* Pt[4] = {pr.dP[0], pr.dP[1], pr.dP[2], pr.dP[3]};
         const double tiles = (double)syrk_packed_tiles(pr.nblk, 0, jt, pr.nblk, 0, 1);
